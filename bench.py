@@ -514,13 +514,17 @@ def ours(args):
                     reference_attention_weight=0.95, audio_attention_weight=3.0, do_multi_devices_inference=dist)
 
     def timed(fn, k):
+        """-> (device seconds, wall seconds, launches, result of the last of the k calls)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = _ffi.LAUNCHES
+        out = None
         t0 = time.perf_counter()
         e0.record()
-        for _ in range(k):
-            fn()
+        for i in range(k):
+            out = fn()
+            if i + 1 < k:
+                out = None          # release a step's result before the next step allocates its own
         e1.record()
         barrier()
         wall = time.perf_counter() - t0
@@ -528,13 +532,16 @@ def ours(args):
         t = torch.tensor([ms, wall * 1e3], device=dev)
         if dist:
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
-        return t[0].item() / 1e3, t[1].item() / 1e3, _ffi.LAUNCHES - l0
+        return t[0].item() / 1e3, t[1].item() / 1e3, _ffi.LAUNCHES - l0, out
 
     for _ in range(args.warmup):
         resident_pass()
     with Clocks(local) as clk:
-        sec, _, launches_direct = timed(resident_pass, args.steps)
+        sec, _, launches_direct, video = timed(resident_pass, args.steps)
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, video=video)
+    del video
     if os.environ.get("VX_NCU_REGION"):
         # `ncu --profile-from-start off ... python bench.py`: exactly one more pass of the same timed workload
         torch.cuda.synchronize()
@@ -562,7 +569,7 @@ def ours(args):
 
     for _ in range(max(1, min(args.warmup, 1))):
         e2e_pass()
-    _, e2e_wall, _ = timed(e2e_pass, args.steps)
+    _, e2e_wall, _, _ = timed(e2e_pass, args.steps)
 
     reader.update(pipe.reference_net.writer_view, True, dtype=torch.bfloat16)   # the pipeline call cleared the banks
 
@@ -662,6 +669,27 @@ def pipe_decode_device(pipe, latents, dist):
     return pipe.decode_to_device(latents, dist)
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, **arrays):
+    """--dump-outputs DIR: every array as DIR/<name>.npy in float32, so that two builds run with the same arguments
+    (hence the same seeded inputs) can be compared output for output.  When the arrays exceed DUMP_LIMIT_BYTES in all,
+    each is replaced by the same fixed, seeded sample of its flattened elements (drawn with replacement; the indices
+    depend only on the element count, so runs with the same arguments sample the same positions)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values())
+    keep = (DUMP_LIMIT_BYTES - 4096 * len(arrays)) // 4          # float32 elements that fit, 4 KB per .npy header
+    for name, a in arrays.items():
+        shape, a = tuple(a.shape), a.detach().float()
+        if total > keep:
+            idx = torch.randint(a.numel(), (keep * a.numel() // total,), generator=torch.Generator().manual_seed(0))
+            a = a.reshape(-1)[idx.to(a.device)]
+        np.save(os.path.join(path, f"{name}.npy"), a.cpu().numpy())
+        sys.stderr.write(f"bench.py: {name} {shape} -> {os.path.join(path, name)}.npy {tuple(a.shape)}\n")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -671,7 +699,12 @@ def main():
     ap.add_argument("--frames", type=int, default=0, help="video length override (multiple of 8, >= 16): 96 = configs[2], 384 = configs[3]")
     ap.add_argument("--size", type=int, default=512, help="video side in pixels (512, or 768 = configs[4])")
     ap.add_argument("--ddim-steps", type=int, default=25)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the video of the last one to DIR/video.npy (float32, a seeded "
+                         "sample when above 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arm only")
     global FRAMES_OVERRIDE, LATENT, DDIM_STEPS
     FRAMES_OVERRIDE, LATENT, DDIM_STEPS = args.frames, args.size // 8, args.ddim_steps
     if args.impl == "reference":

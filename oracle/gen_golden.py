@@ -14,8 +14,13 @@ Inputs/weights are NOT stored: they are regenerated from seeds by ``oracle.vx_or
   * ``modules/v_kps_guider.py``, ``modules/audio_projection.py``, the audio windowing of
      ``VExpressPipeline.prepare_audio_embeddings`` and ``median_filter_3d`` of ``pipelines/utils.py`` (SURVEY 8f-f2/f3;
      the latter executed from its source because the module imports cv2 / ffmpeg)      -> prologue_small.pt
+  * parameter names / defaults of the public entry points the product mirrors (read with ``ast``)
+                                                                               -> reference_signatures.json
 
-Usage:  python oracle/gen_golden.py [context ddim unet pipeline refnet prologue]   (default: all)
+The largest outputs (UNet taps, decoded video) are stored as every SAMPLE_STRIDE-th element of the flattened tensor, with
+the full shape beside them, so that every golden file stays under 1 MB.
+
+Usage:  python oracle/gen_golden.py [context ddim unet pipeline refnet prologue signatures]   (default: all)
 """
 import importlib
 import importlib.util
@@ -33,6 +38,7 @@ sys.path.insert(0, os.path.join(ROOT, "oracle", "diffusers_shim"))
 from oracle import vx_oracle as O  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+SAMPLE_STRIDE = 3       # odd, so the sample walks through every column / row parity of the power-of-two image sides
 
 
 def import_reference():
@@ -145,8 +151,9 @@ def gen_unet(msa, unet3d):
             hk.remove()
         out2 = model(x, 959, encoder_hidden_states=enc, kps_features=kps, return_dict=False)[0]
     torch.save(dict(cfg=cfg, seed_weights=1234, seed_inputs=42, f=f, h=h, ref_w=0.95, audio_w=3.0,
-                    bank_order=order, out_t499=out, out_t959=out2,
-                    taps={k: v.half() for k, v in taps.items()}),
+                    bank_order=order, out_t499=out, out_t959=out2, sample_stride=SAMPLE_STRIDE,
+                    tap_shapes={k: tuple(v.shape) for k, v in taps.items()},
+                    taps={k: v.flatten()[::SAMPLE_STRIDE].half() for k, v in taps.items()}),
                os.path.join(GOLD, "unet_small.pt"))
     print("unet_small.pt: out", tuple(out.shape), "absmean", out.abs().mean().item())
 
@@ -220,7 +227,8 @@ def gen_pipeline(msa, unet3d, pipe, L=12, S=8, Ov=4, steps=3, name="pipeline_sma
         msa.ReferenceAttentionControl.update = real_update
     out = dict(cfg=cfg, vae_cfg=vcfg, L=L, h=h, S=S, O=Ov, steps=steps, guidance_scale=gs, final_latents=captured["latents"])
     if with_video:
-        out["video"] = video.half()
+        out.update(video_shape=tuple(video.shape), sample_stride=SAMPLE_STRIDE,
+                   video=video.flatten()[::SAMPLE_STRIDE].half())
     torch.save(out, os.path.join(GOLD, name))
     print(name, ": video", tuple(video.shape), "latents absmean", captured["latents"].abs().mean().item())
 
@@ -348,11 +356,58 @@ def gen_ddim():
     print("ddim_kat.json", kat["step_t999_n25"])
 
 
+SIGNATURES = [  # (reference file, class, function): the drop-in boundary the product keeps
+    ("pipelines/v_express_pipeline.py", "VExpressPipeline", "__call__"),
+    ("pipelines/v_express_pipeline.py", "VExpressPipeline", "mean_overlap"),
+    ("pipelines/v_express_pipeline.py", "VExpressPipeline", "__init__"),
+    ("pipelines/v_express_pipeline.py", "VExpressPipeline", "prepare_reference_latent"),
+    ("pipelines/v_express_pipeline.py", "VExpressPipeline", "prepare_kps_feature"),
+    ("pipelines/v_express_pipeline.py", "VExpressPipeline", "prepare_audio_embeddings"),
+    ("modules/unet_3d.py", "UNet3DConditionModel", "forward"),
+    ("modules/unet_3d.py", "UNet3DConditionModel", "from_config_2d"),
+    ("modules/unet_3d.py", "UNet3DConditionModel", "__init__"),
+    ("modules/mutual_self_attention.py", "ReferenceAttentionControl", "__init__"),
+    ("modules/mutual_self_attention.py", "ReferenceAttentionControl", "update"),
+    ("modules/mutual_self_attention.py", "ReferenceAttentionControl", "clear"),
+    ("pipelines/context.py", None, "uniform"),
+    ("pipelines/context.py", None, "get_context_scheduler"),
+    ("pipelines/context.py", None, "ordered_halving"),
+]
+
+
+def ast_signature(path, cls, fn):
+    """[(name, default source or '<required>')] of a function in a source file, without importing it."""
+    import ast
+    tree = ast.parse(open(path).read())
+    body = tree.body
+    if cls is not None:
+        body = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == cls).body
+    f = next(n for n in body if isinstance(n, (ast.FunctionDef, ast.AsyncFunctionDef)) and n.name == fn)
+    a = f.args
+    pos = a.posonlyargs + a.args
+    defaults = [None] * (len(pos) - len(a.defaults)) + list(a.defaults)
+    out = []
+    for arg, d in zip(pos, defaults):
+        out.append((arg.arg, "<required>" if d is None else ast.unparse(d)))
+    for arg, d in zip(a.kwonlyargs, a.kw_defaults):
+        out.append((arg.arg, "<required>" if d is None else ast.unparse(d)))
+    if a.kwarg is not None:
+        out.append(("**" + a.kwarg.arg, ""))
+    return out
+
+
+def gen_signatures():
+    sigs = [dict(file=f, cls=c, fn=fn, params=ast_signature(os.path.join(REF, f), c, fn)) for f, c, fn in SIGNATURES]
+    with open(os.path.join(GOLD, "reference_signatures.json"), "w") as fh:
+        json.dump(sigs, fh, indent=1)
+    print("reference_signatures.json:", len(sigs), "entry points")
+
+
 if __name__ == "__main__":
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(os.cpu_count())
     msa, unet3d, ctx, pipe = import_reference()
-    which = set(sys.argv[1:]) or {"context", "ddim", "unet", "pipeline", "refnet", "prologue"}
+    which = set(sys.argv[1:]) or {"context", "ddim", "unet", "pipeline", "refnet", "prologue", "signatures"}
     if "context" in which:
         gen_context(ctx)
     if "ddim" in which:
@@ -377,3 +432,5 @@ if __name__ == "__main__":
         gen_refnet(msa, unet3d)
     if "prologue" in which:
         gen_prologue(pipe)
+    if "signatures" in which:
+        gen_signatures()

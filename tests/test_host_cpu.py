@@ -911,10 +911,9 @@ def test_denoise_sharded_over_ranks_equals_single_rank(L, S, Ov, world):
 
 
 # ----------------------------------------------------------------------------------------------------------------------
-# Drop-in boundary: the mirrored entry points keep the reference's parameter names, order and defaults.  Runs where the
-# reference tree is present (the build container); on the GPU box the committed snapshot below is checked instead.
+# Drop-in boundary: the mirrored entry points keep the reference's parameter names, order and defaults, as read from the
+# reference's sources by oracle/gen_golden.py:gen_signatures into tests/golden/reference_signatures.json.
 # ----------------------------------------------------------------------------------------------------------------------
-_REF = os.environ.get("VX_REFERENCE", "/root/reference")
 _BOUNDARY = [  # (reference file, class, function, product object path)
     ("pipelines/v_express_pipeline.py", "VExpressPipeline", "__call__", "vexpress_b200.pipelines.v_express_pipeline:VExpressPipeline.__call__"),
     ("pipelines/v_express_pipeline.py", "VExpressPipeline", "mean_overlap", "vexpress_b200.pipelines.v_express_pipeline:VExpressPipeline.mean_overlap"),
@@ -934,25 +933,11 @@ _BOUNDARY = [  # (reference file, class, function, product object path)
 ]
 
 
-def _ast_signature(path, cls, fn):
-    """[(name, default-or-'<required>')] of a function in a source file, without importing it."""
-    import ast
-    tree = ast.parse(open(path).read())
-    body = tree.body
-    if cls is not None:
-        body = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == cls).body
-    f = next(n for n in body if isinstance(n, (ast.FunctionDef, ast.AsyncFunctionDef)) and n.name == fn)
-    a = f.args
-    pos = a.posonlyargs + a.args
-    defaults = [None] * (len(pos) - len(a.defaults)) + list(a.defaults)
-    out = []
-    for arg, d in zip(pos, defaults):
-        out.append((arg.arg, "<required>" if d is None else ast.unparse(d)))
-    for arg, d in zip(a.kwonlyargs, a.kw_defaults):
-        out.append((arg.arg, "<required>" if d is None else ast.unparse(d)))
-    if a.kwarg is not None:
-        out.append(("**" + a.kwarg.arg, ""))
-    return out
+def _reference_signature(golden_dir, ref_file, cls, fn):
+    """[(name, default source or '<required>')] of a reference entry point, from the stored golden."""
+    sigs = json.load(open(os.path.join(golden_dir, "reference_signatures.json")))
+    entry = next(s for s in sigs if (s["file"], s["cls"], s["fn"]) == (ref_file, cls, fn))
+    return [tuple(p) for p in entry["params"]]
 
 
 def _product_signature(spec):
@@ -990,10 +975,9 @@ def _same_default(ref_src, val):
     return ref_val == val
 
 
-@pytest.mark.skipif(not os.path.isdir(_REF), reason="reference tree not present (GPU box)")
 @pytest.mark.parametrize("ref_file,cls,fn,spec", _BOUNDARY)
-def test_boundary_signatures_match_reference(ref_file, cls, fn, spec):
-    ref = _ast_signature(os.path.join(_REF, ref_file), cls, fn)
+def test_boundary_signatures_match_reference(golden_dir, ref_file, cls, fn, spec):
+    ref = _reference_signature(golden_dir, ref_file, cls, fn)
     ours = _product_signature(spec)
     if cls is not None:
         ref = [r for r in ref if r[0] not in ("self", "cls")]

@@ -76,8 +76,10 @@ def test_unet_forward_matches_reference(golden_dir):
         out2 = O.unet_forward(sd, cfg, x, 959, enc, kps, banks, g["ref_w"], g["audio_w"])
     torch.testing.assert_close(out, g["out_t499"], atol=2e-4, rtol=1e-4)
     torch.testing.assert_close(out2, g["out_t959"], atol=2e-4, rtol=1e-4)
+    s = g["sample_stride"]
     for k, v in g["taps"].items():
-        torch.testing.assert_close(taps[k], v.float(), atol=2e-2, rtol=2e-3)   # taps stored in fp16
+        assert tuple(taps[k].shape) == g["tap_shapes"][k], k
+        torch.testing.assert_close(taps[k].flatten()[::s], v.float(), atol=2e-2, rtol=2e-3)   # taps stored in fp16
 
 
 def test_pipeline_matches_reference(golden_dir):
@@ -90,8 +92,8 @@ def test_pipeline_matches_reference(golden_dir):
         final = O.denoise(sd, cfg, lat, kps, audio, banks, g["steps"], g["guidance_scale"], g["S"], g["O"], 0.95, 3.0)
         torch.testing.assert_close(final, g["final_latents"], atol=5e-4, rtol=1e-4)
         video = O.decode_latents(vsd, vcfg, final)
-    assert video.shape == g["video"].shape and video.dtype == torch.float32
-    torch.testing.assert_close(video, g["video"].float(), atol=2e-3, rtol=0)
+    assert tuple(video.shape) == g["video_shape"] and video.dtype == torch.float32
+    torch.testing.assert_close(video.flatten()[::g["sample_stride"]], g["video"].float(), atol=2e-3, rtol=0)
 
 
 def test_pipeline_non_tiling_length_matches_reference(golden_dir):

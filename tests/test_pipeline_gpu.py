@@ -106,9 +106,9 @@ def test_pipeline_vs_reference_golden(golden_dir, use_graph):
                  video_length=g["L"], num_inference_steps=g["steps"], guidance_scale=g["guidance_scale"],
                  context_frames=g["S"], context_overlap=g["O"], reference_attention_weight=0.95,
                  audio_attention_weight=3.0)
-    assert video.shape == g["video"].shape and video.dtype == torch.float32 and video.device.type == "cpu"
+    assert tuple(video.shape) == g["video_shape"] and video.dtype == torch.float32 and video.device.type == "cpu"
     e_lat = _rel(captured["latents"], g["final_latents"])
-    d = (video - g["video"].float()).abs()
+    d = (video.flatten()[::g["sample_stride"]] - g["video"].float()).abs()
     print(f"graph={use_graph} final latents rel {e_lat:.3e}; video mean abs {d.mean().item():.3e} max {d.max().item():.3e}")
     assert e_lat < 6e-2 and d.mean().item() < 1.5e-2
     # a second call on the same pipeline object reuses the captured graph / persistent bank buffers

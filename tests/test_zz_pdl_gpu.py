@@ -88,5 +88,5 @@ def test_pipeline_bit_identical_with_pdl(golden_dir, use_graph, restore_pdl):
                            context_frames=g["S"], context_overlap=g["O"], reference_attention_weight=0.95,
                            audio_attention_weight=3.0))
     assert torch.equal(videos[0], videos[1])
-    d = (videos[1] - g["video"].float()).abs().mean().item()
+    d = (videos[1].flatten()[::g["sample_stride"]] - g["video"].float()).abs().mean().item()
     assert d < 1.5e-2, d

@@ -9,7 +9,7 @@ FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompil
 pids=()
 for f in vx_*.cu; do
   o=build/${f%.cu}.o
-  if [ ! -f $o ] || [ $f -nt $o ] || [ vx_ptx.cuh -nt $o ] || [ vx_host.h -nt $o ] || [ ../../include/vxb200.h -nt $o ]; then
+  if [ ! -f $o ] || [ $f -nt $o ] || [ vx_ptx.cuh -nt $o ] || [ vx_host.h -nt $o ] || [ vx_bringup.h -nt $o ] || [ ../../include/vxb200.h -nt $o ]; then
     ( $NVCC $FLAGS ${VX_PTXAS_V:+-Xptxas -v} -I../../include -c $f -o $o ) &
     pids+=($!)
   fi
